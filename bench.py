@@ -6,7 +6,12 @@ optimization.py:91-104) on synthetic BERT-Small-shaped gradients: N-1 accumulate
 accumulate+clip+AdamWeightDecay apply launch per window of N.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload bert_small]
+                  [--dump-outputs DIR]
   torchrun --nproc-per-node N bench.py --gpus N ...        (one rank per GPU, NCCL)
+
+`--dump-outputs DIR` writes what the last timed micro-step left for its caller as DIR/<name>.npy
+(see dump_outputs); the inputs are seeded, so two builds run with the same arguments can be compared
+output for output.
 
 `value`     : whole-job micro-batches/s with gradients already resident in HBM (all ranks).
 `e2e`       : same metric through the public host-buffer call: gradients start in pinned host
@@ -29,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 WORKLOADS = {
     # name -> (manifest key, default N, description)   BASELINE.json configs
@@ -66,6 +72,37 @@ def set_phase(r: int, R: int, N: int) -> int:
 
 def set_start_step(r: int, R: int, N: int) -> int:
     return START_STEP - START_STEP % N + set_phase(r, R, N)
+
+
+DUMP_SAMPLE = 1 << 21    # elements kept per dumped array: four 8 MB arrays stay well inside 64 MB at any workload size
+
+
+def dump_outputs(out_dir, op, params, dp, rank):
+    """Writes what the last timed micro-step left for its caller, as float32 DIR/<name>.npy: the updated parameters
+    (param), the optimizer state the next micro-step reads (adam_m, adam_v, accum), each flattened in manifest order
+    without the slab padding, and the stats block (stats: applied, lr, global_norm, clip_scale).  Arrays longer than
+    DUMP_SAMPLE keep the same sorted sample of indices, drawn from a fixed seed.  Under data parallelism every rank
+    must call it (the moments are gathered from their shards); rank 0 writes."""
+    import numpy as np
+    import torch
+    state = dp.gather_state() if dp is not None else {"m": op.m, "v": op.v}
+    st = op.stats()
+    if rank != 0:
+        return
+
+    def flat(slab):
+        return torch.cat([slab[o:o + p.numel()] for o, p in zip(op.plan.offsets, params)])
+    arrays = {"param": torch.cat([p.reshape(-1) for p in params]), "adam_m": flat(state["m"]),
+              "adam_v": flat(state["v"]), "accum": flat(op.accum)}
+    n = arrays["param"].numel()
+    idx = None
+    if n > DUMP_SAMPLE:
+        idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE, replace=False))).to(op.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), (a if idx is None else a[idx]).cpu().numpy())
+    np.save(os.path.join(out_dir, "stats.npy"),
+            np.array([st["applied"], st["lr"], st["global_norm"], st["clip_scale"]], dtype=np.float32))
 
 
 def _finite(x):
@@ -367,6 +404,9 @@ def run_b200_arm(args):
     clocks = sampler.stop()
     if dist is not None:
         dist.barrier()
+    if args.dump_outputs:
+        op, params, _, _, dp = sets[(base + K - 1) % R]
+        dump_outputs(args.dump_outputs, op, params, dp, rank)
     total_ms = evs[0].elapsed_time(evs[K])
     per = [evs[i].elapsed_time(evs[i + 1]) for i in range(K)] if not args.no_launch_events else [total_ms / K] * K
     if dist is not None:
@@ -719,7 +759,13 @@ def main():
     ap.add_argument("--parity-steps", type=int, default=-1, help="micro-steps of the pre-timing parity self-check against the CPU oracle (-1: 2*min(N,4)+1, 0: skip)")
     ap.add_argument("--e2e-keep-affinity", action="store_true", help="experiment: keep the GPU-local CPU affinity for the whole e2e leg")
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of CPU-oracle timing (0 disables)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's parameters, optimizer state and stats as DIR/<name>.npy (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200: the reference arm times the CPU oracle, not the train_op")
     args.cpu_budget_given = any(a.startswith("--cpu-budget") for a in sys.argv[1:])
     if args.impl == "reference":
         run_reference_arm(args)

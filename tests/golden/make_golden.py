@@ -1,15 +1,16 @@
 #!/usr/bin/env python
 """Generates tests/golden/ref_optimization_*.npz by EXECUTING THE REFERENCE'S OWN optimization.py.
 
-Runs only in the authoring container (it reads /root/reference, which does not exist on the GPU
-box).  TensorFlow is not installable here, so the reference file is imported unmodified with
-oracle/tf_stub first on sys.path (a numpy fp32 emulation of the TF1 primitives it calls; see that
-package's docstring for exactly what this does and does not pin).  For each case we build the
+Needs a checkout of the upstream project (hpandana/gradient-accumulation-tf-estimator, commit
+74ae92b8) named by GACCUM_REFERENCE_DIR.  TensorFlow is not a dependency of this project, so the
+reference file is imported unmodified with oracle/tf_stub first on sys.path (a numpy fp32 emulation
+of the TF1 primitives it calls; see that package's docstring for exactly what this does and does
+not pin).  For each case we build the
 reference graph with `optimization.create_optimizer(loss, init_lr, num_train_steps,
 num_warmup_steps, use_tpu=False)`, feed seeded gradients for 2*N+2 micro-steps (N = 8, hard-coded
 at optimization.py:76) and record every variable after every `session.run(train_op)`.
 
-    python tests/golden/make_golden.py          # rewrites the fixtures
+    GACCUM_REFERENCE_DIR=<checkout> python tests/golden/make_golden.py          # rewrites the fixtures
 """
 import importlib
 import json
@@ -20,7 +21,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REFERENCE = "/root/reference"
+REFERENCE = os.environ.get("GACCUM_REFERENCE_DIR", "")     # checkout of the upstream project
 
 # mini-BERT: names drive the decay mask (LayerNorm / layer_norm / bias are excluded, :65)
 VARIABLES = [
@@ -102,11 +103,13 @@ def run_case(name, init_lr, num_train_steps, num_warmup_steps, sigma, seed):
 
 if __name__ == "__main__":
     if not os.path.isdir(REFERENCE):
-        raise SystemExit("make_golden.py needs /root/reference (authoring container only)")
+        raise SystemExit("make_golden.py needs GACCUM_REFERENCE_DIR: a checkout of the upstream project")
+    sys.path.insert(0, os.path.dirname(HERE))
+    from golden_util import array_digests
     meta = {}
     for name, cfg in CASES.items():
         path, steps = run_case(name, *cfg)
-        meta[name] = {"file": os.path.basename(path), "steps": steps, "config": cfg}
+        meta[name] = {"file": os.path.basename(path), "steps": steps, "config": cfg, "digests": array_digests(path)}
         print("wrote", path)
     with open(os.path.join(HERE, "MANIFEST.json"), "w") as f:
         json.dump({"generator": "tests/golden/make_golden.py", "reference_commit": "74ae92b8",

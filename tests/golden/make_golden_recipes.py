@@ -1,10 +1,11 @@
 #!/usr/bin/env python
 """Generates tests/golden/ref_recipe_*.npz and the extra ref_optimization_* cases by EXECUTING THE
-REFERENCE'S OWN STATEMENTS, lifted by AST from the files under /root/reference.
+REFERENCE'S OWN STATEMENTS, lifted by AST from the files of the upstream project.
 
-Runs only in the authoring container (it reads /root/reference).  TensorFlow is not installable, so the
-lifted statements run against oracle/tf_stub (numpy fp32 emulation; tests/golden/MANIFEST.json lists which
-stub primitives are restatements of TensorFlow rather than of the reference).
+Needs a checkout of the upstream project (commit 74ae92b8) named by GACCUM_REFERENCE_DIR.  TensorFlow is
+not a dependency of this project, so the lifted statements run against oracle/tf_stub (numpy fp32 emulation;
+tests/golden/MANIFEST.json lists which stub primitives are restatements of TensorFlow rather than of the
+reference).
 
 What is lifted, verbatim (ast nodes selected by line number, compiled, exec'd -- never retyped):
   * distributedExample/02_single_worker_with_estimator_gaccum.py  model_fn lines 38-41 (hyper-parameters,
@@ -22,7 +23,7 @@ N=3; nothing else changes.  A third calls the reference's AdamWeightDecayOptimiz
 with a (None, var) pair, the only way the reference's `if grad is None` branch (optimization.py:132-133) can
 execute (through create_optimizer a None gradient raises in assign_add, in TF and in the stub alike).
 
-    python tests/golden/make_golden_recipes.py          # rewrites the fixtures + MANIFEST entries
+    GACCUM_REFERENCE_DIR=<checkout> python tests/golden/make_golden_recipes.py          # rewrites the fixtures + MANIFEST entries
 """
 import ast
 import importlib
@@ -35,7 +36,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REFERENCE = "/root/reference"
+REFERENCE = os.environ.get("GACCUM_REFERENCE_DIR", "")     # checkout of the upstream project
 SEED0 = 19830610
 
 MNIST = [("conv2d/kernel", (3, 3, 1, 32)), ("conv2d/bias", (32,)), ("dense/kernel", (5408, 64)), ("dense/bias", (64,)),
@@ -246,15 +247,25 @@ def run_optimization_case_full_size(case, N, init_lr, num_train_steps, num_warmu
         else:
             out[key] = arr.copy()
     sess = tf.Session()
+    prev = None
     for s in range(steps):
         gl = grads_for(variables, sigma, seed, s)
         sess.run(train_op, feed_dict={grad_ph[vname + ":0"]: g for (vname, _), g in zip(variables, gl)})
         if s >= steps - 2:
+            cur = {(kind, vname): by_name[vname + sfx].value.copy() for vname, _ in variables
+                   for kind, sfx in (("param", ":0"), ("m", "/adam_m:0"), ("v", "/adam_v:0"))}
+            # an accumulate-only micro-step leaves param / m / v as they were: stored once, under the step before
+            same = prev is not None and all(np.array_equal(cur[k], prev[k]) for k in cur)
+            if same:
+                out[f"same_as/{s}"] = np.int64(s - 1)
             for i, (vname, _) in enumerate(variables):
-                store(f"param/{s}/{vname}", by_name[vname + ":0"].value)
+                if not same:
+                    store(f"param/{s}/{vname}", cur["param", vname])
                 store(f"accum/{s}/{vname}", accum_vars[i].value)
-                store(f"m/{s}/{vname}", by_name[vname + "/adam_m:0"].value)
-                store(f"v/{s}/{vname}", by_name[vname + "/adam_v:0"].value)
+                if not same:
+                    store(f"m/{s}/{vname}", cur["m", vname])
+                    store(f"v/{s}/{vname}", cur["v", vname])
+            prev = cur
         out[f"global_step/{s}"] = np.int64(by_name["global_step:0"].value)
     out["recorded_steps"] = np.array([steps - 2, steps - 1])
     path = os.path.join(HERE, f"ref_fullsize_{case}.npz")
@@ -300,7 +311,9 @@ def run_direct_apply_with_none(case, lr, sigma, seed, steps):
 
 if __name__ == "__main__":
     if not os.path.isdir(REFERENCE):
-        raise SystemExit("make_golden_recipes.py needs /root/reference (authoring container only)")
+        raise SystemExit("make_golden_recipes.py needs GACCUM_REFERENCE_DIR: a checkout of the upstream project")
+    sys.path.insert(0, os.path.dirname(HERE))
+    from golden_util import array_digests
     meta = {}
     ex02 = "distributedExample/02_single_worker_with_estimator_gaccum.py"
     ex04 = "distributedExample/04_multi_worker_with_estimator_gaccum.py"
@@ -336,13 +349,16 @@ if __name__ == "__main__":
     path, edits = run_optimization_case_full_size("bert_small_n4", 4, 2e-5, 207900, 6, 1e-3, 41, 10)
     meta["fullsize_bert_small_n4"] = {"file": os.path.basename(path), "reference_file": "optimization.py",
                                       "edits": [f"line {ln}: literal {old} -> {new} (AST)" for ln, old, new in edits],
-                                      "shapes": "BERT-Small L4_H512 (T=73, P=28 764 674)", "stored": f"last two micro-steps, every {BIG_STRIDE}th element + fp64 sums",
+                                      "shapes": "BERT-Small L4_H512 (T=73, P=28 764 674)", "stored": f"last two micro-steps, every {BIG_STRIDE}th element + fp64 sums; param / m / v of the "
+                                                "accumulate-only last step once, under the step before (same_as/<step>)",
                                       "config": [2e-5, 207900, 6, 1e-3, 41, 10]}
     print("wrote", path)
     path = run_direct_apply_with_none("direct_apply_none_grad", 1e-3, 0.3, 33, 3)
     meta["direct_apply_none_grad"] = {"file": os.path.basename(path), "reference_file": "optimization.py (unmodified)",
                                       "what": "AdamWeightDecayOptimizer.apply_gradients(zip(grads, tvars)) with grads[3] = None (:132-133)"}
     print("wrote", path)
+    for entry in meta.values():
+        entry["digests"] = array_digests(os.path.join(HERE, entry["file"]))
     man_path = os.path.join(HERE, "MANIFEST.json")
     with open(man_path) as fh:
         man = json.load(fh)

@@ -56,6 +56,36 @@ def test_b200_arm_line():
     assert d["parity"]["ok"] is True and d["parity"]["max_rel_err"] <= 1e-5 and d["parity"]["world"] == 1
 
 
+@pytest.mark.gpu
+def test_b200_arm_dumps_the_last_timed_step(tmp_path):
+    """--dump-outputs: float32 arrays within 64 MB, identical for identical arguments, and they follow --steps."""
+    import numpy as np
+    base = ["--workload", "mnist_cnn", "--warmup", "3", "--e2e-steps", "0", "--model-steps", "0", "--cpu-budget", "0",
+            "--parity-steps", "0"]
+    runs = {}
+    for tag, steps in (("a", 8), ("b", 8), ("c", 12)):
+        d = _run(base + ["--steps", str(steps), "--dump-outputs", str(tmp_path / tag)])
+        assert d["steps"] == steps and d["config"]["apply_launches"] == steps // 4
+        runs[tag] = {n: np.load(tmp_path / tag / f"{n}.npy") for n in ("param", "adam_m", "adam_v", "accum", "stats")}
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a")) <= 64 << 20
+    a, b, c = runs["a"], runs["b"], runs["c"]
+    P = d["config"]["P"]
+    for n in ("param", "adam_m", "adam_v", "accum"):
+        assert a[n].dtype == np.float32 and a[n].shape == (P,)
+    assert a["stats"].dtype == np.float32 and a["stats"][0] == 1.0      # 8 steps at N=4 end on an apply
+    assert not a["accum"].any()                                            # ... which zeroes the accumulators
+    for n in a:
+        assert np.array_equal(a[n], b[n]), n
+    assert not np.array_equal(a["param"], c["param"])                     # one more window moved the parameters
+
+
+def test_dump_outputs_and_steps_are_validated():
+    for args in (["--impl", "reference", "--dump-outputs", "out"], ["--steps", "0"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + args, capture_output=True, text=True,
+                           timeout=120, cwd=ROOT)
+        assert r.returncode == 2 and "error" in r.stderr and r.stdout == ""
+
+
 def test_both_arms_print_the_same_metric_string():
     """The driver divides the two arms only when `metric` matches: one constant feeds both lines."""
     import re

@@ -1,21 +1,40 @@
-"""The committed golden fixtures are exactly what tests/golden/make_golden.py produces from the
-reference's own optimization.py (only checkable where /root/reference exists: the authoring container)."""
+"""The committed golden fixtures are exactly what tests/golden/make_golden.py and make_golden_recipes.py produce
+from the reference's own code.  The upstream project's source is not part of this repository, so the generators
+record, from their run against it, a sha256 per key family of every fixture in MANIFEST.json: every committed
+fixture is held to those digests.  With GACCUM_REFERENCE_DIR naming a checkout of the upstream project, the
+generators also run again here and must reproduce the committed fixtures bit for bit."""
+import glob
 import importlib.util
+import json
 import os
 import sys
 
 import numpy as np
-import pytest
+
+from golden_util import array_digests
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE = "/root/reference/optimization.py"
+REFERENCE_DIR = os.environ.get("GACCUM_REFERENCE_DIR", "")
+HAVE_REFERENCE = bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "optimization.py"))
+with open(os.path.join(HERE, "golden", "MANIFEST.json")) as _f:
+    MANIFEST = json.load(_f)
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE), reason="/root/reference is not present (GPU box)")
+def _holds_recorded_run(section):
+    for name, e in MANIFEST[section].items():
+        got = array_digests(os.path.join(HERE, "golden", e["file"]))
+        assert got == e["digests"], f"{name}: {e['file']} differs from the upstream run in " + \
+            str(sorted(k for k in set(got) | set(e["digests"]) if got.get(k) != e["digests"].get(k)))
+
+
 def test_fixtures_regenerate_bit_identically(tmp_path, monkeypatch):
     spec = importlib.util.spec_from_file_location("make_golden", os.path.join(HERE, "golden", "make_golden.py"))
     mg = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mg)
+    assert set(MANIFEST["cases"]) == set(mg.CASES)
+    _holds_recorded_run("cases")
+    if not HAVE_REFERENCE:
+        return
     monkeypatch.setattr(mg, "HERE", str(tmp_path))
     saved_path, saved_mods = list(sys.path), {k: sys.modules.get(k) for k in ("tensorflow", "optimization")}
     try:
@@ -35,10 +54,15 @@ def test_fixtures_regenerate_bit_identically(tmp_path, monkeypatch):
                 sys.modules[k] = v
 
 
-@pytest.mark.skipif(not os.path.exists(REFERENCE), reason="/root/reference is not present (GPU box)")
 def test_recipe_fixtures_regenerate_bit_identically(tmp_path, monkeypatch):
     """Same for tests/golden/make_golden_recipes.py: the AST-lifted statements of 02 / 04 / another-example and the
-    N-patched optimization.py produce exactly the committed ref_recipe_* / ref_optimization_n* / ref_direct_* files."""
+    N-patched optimization.py produce exactly the committed ref_recipe_* / ref_optimization_n* / ref_direct_* /
+    ref_fullsize_* files; between them, the two generators' records cover every committed fixture."""
+    recorded = {e["file"] for sec in ("cases", "recipe_cases") for e in MANIFEST[sec].values()}
+    assert recorded == {os.path.basename(p) for p in glob.glob(os.path.join(HERE, "golden", "*.npz"))}
+    _holds_recorded_run("recipe_cases")
+    if not HAVE_REFERENCE:
+        return
     spec = importlib.util.spec_from_file_location("make_golden_recipes", os.path.join(HERE, "golden", "make_golden_recipes.py"))
     mg = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mg)
