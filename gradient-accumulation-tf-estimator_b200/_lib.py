@@ -74,13 +74,8 @@ def _load():
     global _lib
     if _lib is not None:
         return _lib
-    override = os.environ.get("GACCUM_LIB")    # measurement builds (build.build_variant), never a fallback
-    if override:
-        if not os.path.exists(override):
-            raise ImportError(f"GACCUM_LIB={override} does not exist")
-        _build.LIB = override
     try:
-        path = override or _build.build_libgaccum()
+        path = _build.build_libgaccum()
     except Exception as e:  # no nvcc and no prebuilt library: fail loudly, never fall back
         if not os.path.exists(_build.LIB):
             raise ImportError(f"libgaccum.so is missing and cannot be built ({e}); "

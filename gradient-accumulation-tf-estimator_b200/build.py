@@ -43,20 +43,5 @@ def build_libgaccum(force: bool = False, verbose: bool = False) -> str:
     return LIB
 
 
-def build_variant(name: str, defines, verbose: bool = False) -> str:
-    """A/B builds for measurement only (tools/): csrc/libgaccum_<name>.so with extra -D flags, e.g. the
-    experiments build (-DGACCUM_EXPERIMENTS: per-CTA timestamps).  Loaded through GACCUM_LIB=<path>."""
-    out = os.path.join(CSRC, f"libgaccum_{name}.so")
-    cmd = [nvcc_path()] + NVCC_FLAGS + [f"-D{d}" for d in defines] + (["-Xptxas", "-v"] if verbose else []) + ["-o", out] + SOURCES
-    env = dict(os.environ)
-    env.pop("CC", None); env.pop("CXX", None)
-    subprocess.check_call(cmd, cwd=CSRC, env=env)
-    return out
-
-
 if __name__ == "__main__":
-    import sys
-    if len(sys.argv) > 2 and sys.argv[1] == "--variant":
-        print(build_variant(sys.argv[2], sys.argv[3:], verbose=False))
-    else:
-        print(build_libgaccum(force=True, verbose=True))
+    print(build_libgaccum(force=True, verbose=True))

@@ -7,7 +7,6 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <mutex>
@@ -58,22 +57,15 @@ struct gaccum_plan {
   int64_t P = 0, padded = 0;
   // device side
   TileDesc* d_tiles = nullptr;
-  double* d_partials = nullptr;
+  double* d_partials = nullptr;           // data-parallel kernel: one norm partial per block
   float* d_stats = nullptr;
   uint32_t* d_dp_sync = nullptr;           // data-parallel kernel: block-completion counters and tile tickets (zero between launches)
   unsigned long long* d_barrier = nullptr; // clip-apply kernel: monotonic arrival counter of the consumers' grid barrier
   LaunchCounters* d_counters = nullptr;    // ... two sets of per-launch counters (tickets, pool length, norm accumulator)
-  bool p1_dynamic = false;                 // ... pass 1 hands out the non-parked tiles by atomic tickets (long passes) or by position (short ones)
-  int tmem_tiles = kTmemTiles;             // tiles of a' per consumer group parked in Tensor Memory (GACCUM_TMEM_TILES: A/B)
-#ifdef GACCUM_EXPERIMENTS
-  unsigned long long* d_debug = nullptr;   // per-CTA timestamps (tools/cta_timeline.py; experiments build only)
-#endif
   int num_sms = 0;
   int max_grid = 0;
-  uint32_t flags = 0;  // kFlag* bits; GACCUM_FLAGS selects A/B measurement variants (all compute the same result)
   std::mutex mu;
   std::map<const void*, int> grid_cache;   // kernel -> co-resident grid size
-  int smem_per_sm = 0, smem_optin = 0;
 };
 
 static int build_layout(gaccum_plan* pl) {
@@ -156,7 +148,7 @@ static int grid_for(gaccum_plan* pl, const void* fn, int* out) {
 }
 
 template <int CAP>
-static int launch_accumulate(gaccum_plan* pl, KernelParams<CAP>& prm, cudaStream_t st) {
+static int launch_accumulate(KernelParams<CAP>& prm, cudaStream_t st) {
   // one tile per CTA: the hardware block scheduler balances better than a persistent loop (r01_tune_sweep.md)
   const int grid = std::max(1, prm.num_tiles);
   accumulate_kernel<CAP><<<grid, kThreads, 0, st>>>(prm);
@@ -165,7 +157,7 @@ static int launch_accumulate(gaccum_plan* pl, KernelParams<CAP>& prm, cudaStream
 }
 
 template <int VARIANT, bool HAS_G, int CAP>
-static int launch_apply_noclip(gaccum_plan* pl, KernelParams<CAP>& prm, cudaStream_t st) {
+static int launch_apply_noclip(KernelParams<CAP>& prm, cudaStream_t st) {
   const int grid = std::max(1, prm.num_tiles);
   apply_kernel<VARIANT, HAS_G, CAP><<<grid, kThreads, 0, st>>>(prm);
   CUDA_TRY(cudaGetLastError());
@@ -191,8 +183,6 @@ static int launch_apply_clip(gaccum_plan* pl, KernelParams<CAP>& prm, cudaStream
   const int grid = std::max(1, std::min(pl->num_sms, ((int)pl->tiles.size() + kGroups - 1) / kGroups));
   prm.barrier = pl->d_barrier;
   prm.counters = pl->d_counters;
-  if (pl->p1_dynamic) prm.flags |= kFlagDynamicPass1;
-  prm.tmem_tiles = pl->tmem_tiles;
   void* args[] = {(void*)&prm};
   CUDA_TRY(cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kClipThreads), args, (size_t)kRingBytes, st));
   return GACCUM_OK;
@@ -203,12 +193,12 @@ static int launch_apply(gaccum_plan* pl, KernelParams<CAP>& prm, bool has_g, cud
   const bool clip = pl->hp.clip_norm > 0.0;
   const int key = (pl->hp.variant == GACCUM_ADAM ? 4 : 0) | (clip ? 2 : 0) | (has_g ? 1 : 0);
   switch (key) {
-    case 0: return launch_apply_noclip<0, false>(pl, prm, st);
-    case 1: return launch_apply_noclip<0, true>(pl, prm, st);
+    case 0: return launch_apply_noclip<0, false>(prm, st);
+    case 1: return launch_apply_noclip<0, true>(prm, st);
     case 2: return launch_apply_clip<0, false>(pl, prm, st);
     case 3: return launch_apply_clip<0, true>(pl, prm, st);
-    case 4: return launch_apply_noclip<1, false>(pl, prm, st);
-    case 5: return launch_apply_noclip<1, true>(pl, prm, st);
+    case 4: return launch_apply_noclip<1, false>(prm, st);
+    case 5: return launch_apply_noclip<1, true>(prm, st);
     case 6: return launch_apply_clip<1, false>(pl, prm, st);
     default: return launch_apply_clip<1, true>(pl, prm, st);
   }
@@ -234,12 +224,7 @@ static void fill_common(gaccum_plan* pl, KernelParams<CAP>& prm, float* accum, f
   prm.accum = accum;
   prm.m = m;
   prm.v = v;
-  prm.partials = pl->d_partials;
-#ifdef GACCUM_EXPERIMENTS
-  prm.debug = pl->d_debug;
-#endif
   prm.stats = pl->d_stats;
-  prm.flags = pl->flags;
   prm.sc = sc;
 }
 
@@ -267,13 +252,12 @@ struct DeviceGuard {
 
 template <int CAP>
 static int do_accumulate_tab(gaccum_plan* pl, const float* const* grads, float* accum,
-                             const gaccum_step_args* a, cudaStream_t st, uint32_t extra_flags = 0) {
+                             const gaccum_step_args* a, cudaStream_t st) {
   KernelParams<CAP>* prm = new (std::nothrow) KernelParams<CAP>();
   if (!prm) return fail(GACCUM_ENOMEM, "out of host memory");
   fill_common(pl, *prm, accum, nullptr, nullptr, make_scalars(pl->hp, a));
-  prm->flags |= extra_flags;
   int rc = fill_table(pl, prm->tab, grads, nullptr);
-  if (rc == GACCUM_OK) rc = launch_accumulate(pl, *prm, st);
+  if (rc == GACCUM_OK) rc = launch_accumulate(*prm, st);
   delete prm;
   return rc;
 }
@@ -299,9 +283,6 @@ static int check_args(const gaccum_step_args* a) {
 
 static void free_plan_device(gaccum_plan* pl) {
   cudaFree(pl->d_tiles); cudaFree(pl->d_partials); cudaFree(pl->d_stats); cudaFree(pl->d_dp_sync); cudaFree(pl->d_barrier); cudaFree(pl->d_counters);
-#ifdef GACCUM_EXPERIMENTS
-  cudaFree(pl->d_debug);
-#endif
 }
 
 // ------------------------------------------------------------------------------------------
@@ -395,13 +376,6 @@ int gaccum_plan_create(gaccum_plan** out, int32_t T, const int64_t* numels, cons
   if (hp->variant == GACCUM_ADAM_WEIGHT_DECAY && decay) pl->decay.assign(decay, decay + T);
   if (int rc = build_layout(pl)) { delete pl; return rc; }
   pl->device = -1;
-  // GACCUM_TMEM_TILES: A/B measurement knob of the clip-apply kernel (how many a' tiles per group are parked in
-  // Tensor Memory); every value computes the same result.  Result-changing timing experiments do not exist in this build.
-  if (const char* t = getenv("GACCUM_TMEM_TILES")) pl->tmem_tiles = std::max(0, std::min(kTmemTiles, atoi(t)));
-  // measured on the same GPU (profiles/r02_tune_sweep.md): handing pass 1's non-parked tiles out by tickets is as fast as
-  // the static split at BERT-Small (176.5 vs 177.0 us) and 1.5-2 % faster at BERT-Base / -Large; GACCUM_P1_DYNAMIC=0 is the A/B knob
-  pl->p1_dynamic = true;
-  if (const char* t = getenv("GACCUM_P1_DYNAMIC")) pl->p1_dynamic = atoi(t) != 0;
   if (device >= 0) {
     int n = gaccum_device_count();
     if (device >= n) { delete pl; return fail(GACCUM_ENODEVICE, "CUDA device %d requested but %d device(s) visible; libgaccum has no CPU fallback", device, n); }
@@ -411,23 +385,17 @@ int gaccum_plan_create(gaccum_plan** out, int32_t T, const int64_t* numels, cons
     if (e == cudaSuccess && !prop.cooperativeLaunch) e = cudaErrorNotSupported;
     const size_t tb = std::max<size_t>(1, pl->tiles.size()) * sizeof(TileDesc);
     pl->num_sms = prop.multiProcessorCount;
-    pl->smem_per_sm = (int)prop.sharedMemPerMultiprocessor;
-    pl->smem_optin = (int)prop.sharedMemPerBlockOptin;
     pl->max_grid = pl->num_sms * 16;
     if (e == cudaSuccess) e = cudaMalloc(&pl->d_tiles, tb);
     if (e == cudaSuccess && !pl->tiles.empty())
       e = cudaMemcpy(pl->d_tiles, pl->tiles.data(), pl->tiles.size() * sizeof(TileDesc), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc(&pl->d_partials, sizeof(double) * std::max<size_t>((size_t)pl->max_grid, pl->tiles.size()));   // per CTA (clip-apply) / per tile (data-parallel apply)
+    if (e == cudaSuccess) e = cudaMalloc(&pl->d_partials, sizeof(double) * (size_t)pl->max_grid);
     if (e == cudaSuccess) e = cudaMalloc(&pl->d_dp_sync, sizeof(uint32_t) * 8);
     if (e == cudaSuccess) e = cudaMemset(pl->d_dp_sync, 0, sizeof(uint32_t) * 8);
     if (e == cudaSuccess) e = cudaMalloc(&pl->d_barrier, sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMemset(pl->d_barrier, 0, sizeof(unsigned long long));
     if (e == cudaSuccess) e = cudaMalloc(&pl->d_counters, 2 * sizeof(LaunchCounters));
     if (e == cudaSuccess) e = cudaMemset(pl->d_counters, 0, 2 * sizeof(LaunchCounters));
-#ifdef GACCUM_EXPERIMENTS
-    if (e == cudaSuccess) e = cudaMalloc(&pl->d_debug, sizeof(unsigned long long) * 16 * (size_t)pl->max_grid);
-    if (e == cudaSuccess) e = cudaMemset(pl->d_debug, 0, sizeof(unsigned long long) * 16 * (size_t)pl->max_grid);
-#endif
     if (e == cudaSuccess) e = cudaMalloc(&pl->d_stats, sizeof(gaccum_stats));
     if (e == cudaSuccess) e = cudaMemset(pl->d_stats, 0, sizeof(gaccum_stats));
     if (e != cudaSuccess) {
@@ -516,7 +484,7 @@ int gaccum_step_packed(gaccum_plan* pl, const float* grad_slab, float* param_sla
   prm.tab.p = param_slab;
   if (!apply) {
     if (!grad_slab) return fail(GACCUM_EINVAL, "grad_slab is NULL on an accumulate step");
-    return launch_accumulate(pl, prm, st);
+    return launch_accumulate(prm, st);
   }
   if (!param_slab || !aligned16_host(param_slab)) return fail(GACCUM_EINVAL, "param_slab must be a 16-byte aligned device pointer");
   return launch_apply(pl, prm, grad_slab != nullptr, st);
@@ -596,9 +564,6 @@ static int do_apply_dp(gaccum_plan* pl, const gaccum_dp_comm* comm, const float*
   prm->partials = pl->d_partials;
   prm->stats = pl->d_stats;
   prm->sync = pl->d_dp_sync;
-#ifdef GACCUM_EXPERIMENTS
-  prm->debug = pl->d_debug;
-#endif
   prm->sc = make_scalars(pl->hp, a);
   prm->rank = comm->rank;
   prm->world = W;
@@ -608,7 +573,6 @@ static int do_apply_dp(gaccum_plan* pl, const gaccum_dp_comm* comm, const float*
   int grid = 0;
   int rc = grid_for(pl, fn, &grid);
   if (rc == GACCUM_OK) {
-    if (const char* t = getenv("GACCUM_DP_BLOCKS_PER_SM")) grid = std::min(grid, std::max(1, atoi(t)) * pl->num_sms);   // A/B knob
     grid = std::max(1, std::min(grid, prm->num_tiles));
     void* args[] = {(void*)prm};
     cudaError_t e = cudaLaunchCooperativeKernel(fn, dim3(grid), dim3(kThreads), args, 0, st);
@@ -878,16 +842,6 @@ int gaccum_host_session_slabs(gaccum_host_session* s, float** out) {
   out[0] = s->d_params; out[1] = s->d_accum; out[2] = s->d_m; out[3] = s->d_v;
   return GACCUM_OK;
 }
-
-#ifdef GACCUM_EXPERIMENTS
-// Experiments build only (-DGACCUM_EXPERIMENTS, not declared in gaccum.h): per-CTA timestamps of the last clip-apply launch.
-extern "C" __attribute__((visibility("default"))) int gaccum_debug_read(gaccum_plan* pl, unsigned long long* out, int n) {
-  if (!pl || !pl->d_debug) return fail(GACCUM_EINVAL, "no debug buffer");
-  DeviceGuard guard(pl->device);
-  CUDA_TRY(cudaMemcpy(out, pl->d_debug, sizeof(unsigned long long) * (size_t)std::min(n, 16 * pl->max_grid), cudaMemcpyDeviceToHost));
-  return GACCUM_OK;
-}
-#endif
 
 int gaccum_read_stats(gaccum_plan* pl, gaccum_stats* host_out, gaccum_stream_t stream) {
   if (!pl || !host_out) return fail(GACCUM_EINVAL, "bad arguments to gaccum_read_stats");

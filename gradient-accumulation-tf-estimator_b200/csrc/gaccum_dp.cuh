@@ -64,9 +64,6 @@ struct DpParams {
   double* partials;
   float* stats;
   uint32_t* sync;                       // [0..2] block-completion counters, [3], [5] tile tickets of phases A and C; zero between launches
-#ifdef GACCUM_EXPERIMENTS
-  unsigned long long* debug;            // 16 timestamps (ns) per block (tools/dp_timeline.py)
-#endif
   Scalars sc;
   int32_t rank, world;
   uint32_t epoch;
@@ -94,9 +91,6 @@ __device__ __forceinline__ void dp_phase_done(const DpParams<CAP>& prm, int phas
   if (threadIdx.x == 0) {
     __threadfence_system();
     s_last = atomicAdd(prm.sync + phase, 1u) == gridDim.x - 1;
-#ifdef GACCUM_EXPERIMENTS
-    if (prm.debug && phase == 1) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); prm.debug[blockIdx.x * 16 + 9] = t; }
-#endif
   }
   __syncthreads();
   if (s_last) {                                // block-uniform
@@ -110,9 +104,6 @@ __device__ __forceinline__ void dp_phase_done(const DpParams<CAP>& prm, int phas
     if (threadIdx.x == 0) {
       __threadfence_system();
       for (int w = 0; w < prm.world; ++w) st_release_sys(prm.ctrl[w] + phase * kMaxRanks + prm.rank, prm.epoch);
-#ifdef GACCUM_EXPERIMENTS
-      if (prm.debug && phase == 1) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); prm.debug[blockIdx.x * 16 + 10] = t; }
-#endif
     }
   }
 }
@@ -331,6 +322,23 @@ __device__ __forceinline__ void dp_update_tile(const TileDesc d, const DpParams<
   }
 }
 
+// Deterministic CTA reduction of one double per thread -> total in thread 0.  Threads add each
+// tile's 8-element fp32 partial into an fp64 running sum, so the norm of a 335 M-element model is
+// good to ~1e-7 relative even for adversarial (constant) data.
+__device__ __forceinline__ double block_reduce_to_double(double x, double* smem /* blockDim.x/32 */) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  if (lane == 0) smem[warp] = x;
+  __syncthreads();
+  double tot = 0.0;
+  if (threadIdx.x == 0) {
+    const int nw = ((int)blockDim.x + 31) >> 5;
+    for (int w = 0; w < nw; ++w) tot += smem[w];
+  }
+  return tot;
+}
+
 template <int VARIANT, int CAP>
 __global__ void __launch_bounds__(kThreads, 4)
 dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
@@ -339,18 +347,6 @@ dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
   const uint64_t pol = policy_evict_last();
   const int W = prm.world, R = prm.rank, nt = prm.num_tiles;
   const int lo = prm.bounds[R], hi = prm.bounds[R + 1];
-#ifdef GACCUM_EXPERIMENTS
-  auto stamp = [&](int which) {
-    if (prm.debug && threadIdx.x == 0) {
-      unsigned long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      prm.debug[blockIdx.x * 16 + which] = t;
-    }
-  };
-#else
-  auto stamp = [](int) {};
-#endif
-  stamp(0);
 
   __shared__ int s_ticket[3];
   TicketLoop tl;
@@ -383,11 +379,8 @@ dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
       t = tn; d = dn;
     }
   }
-  stamp(1);
   dp_phase_done(prm, 0, [] {});
-  stamp(2);
   dp_wait(prm, 0);
-  stamp(3);
 
   // ---- phase B: reduction of the owned shard in fixed rank order + norm partial.  Local traffic only and short: a static
   //      split (block b takes owned tiles b, b + G, ...) beats tickets here (31 vs 48 us at W=2: per-tile barriers
@@ -408,7 +401,6 @@ dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
     const double part = block_reduce_to_double(acc, red);
     if (threadIdx.x == 0) prm.partials[blockIdx.x] = part;
   }
-  stamp(4);
   dp_phase_done(prm, 1, [&] {
     // last block of this rank: per-block partials, fixed tree -> this rank's partial norm -> every rank
     double tot = 0.0;
@@ -422,7 +414,6 @@ dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
     }
   });
   dp_wait(prm, 1);
-  stamp(5);
   if (threadIdx.x == 0) {
     const double* slots = reinterpret_cast<const double*>(reinterpret_cast<const char*>(prm.ctrl[R]) + kCtrlNormByteOffset);
     double tot = 0.0;
@@ -455,11 +446,9 @@ dp_apply_kernel(const __grid_constant__ DpParams<CAP> prm) {
       d = dn;
     }
   }
-  stamp(6);
   dp_phase_done(prm, 2, [] {});
   // every peer's parameter stores into my slab are complete before the kernel ends
   if (blockIdx.x == 0) dp_wait(prm, 2);
-  stamp(7);
 }
 
 }  // namespace gaccum

@@ -7,23 +7,8 @@
 //                        one tile per CTA (hardware block scheduler)
 //   apply_kernel         the apply branch WITHOUT clipping (plain Adam of the example scripts, or
 //                        clip_norm <= 0): a' = a + G; n = a'/N; Adam; a = 0 in a single pass (36 B/elem).
-//   apply_clip_kernel    the apply branch WITH tf.clip_by_global_norm                  (36 B/elem)
-//                        optimization.py:80-88, 128-177.  The global norm of ALL tensors is needed before
-//                        ANY element can be updated, so it is one cooperative launch, one CTA per SM, with
-//                        two passes around a grid barrier:
-//                          pass 1  PRODUCER WARPS stream G into shared-memory tile slots with TMA bulk
-//                                  copies (cp.async.bulk + mbarrier complete_tx; descriptors and L2
-//                                  prefetches of a run ahead), three 256-thread CONSUMER GROUPS load a,
-//                                  take G out of the slots, a' = a + G, reduce sum((a'/N)^2)
-//                                  (thread fp32 per tile -> fp64 running sum -> warp shuffle -> shared
-//                                  memory -> one fp64 partial per CTA); a' is PARKED ON CHIP: the first
-//                                  tiles in Tensor Memory (tcgen05.st), the last ones in the very slots
-//                                  their G landed in (the ring becomes the stash), the rest written back
-//                                  in place tagged L2::evict_last
-//                          barrier every CTA adds the per-CTA partials in the same order
-//                                  (bit-identical gn and clip scale everywhere)
-//                          pass 2  L2-resident tiles youngest first, then the slots, then Tensor Memory:
-//                                  clip, AdamWeightDecay/Adam, write p, m, v, a = 0
+//   apply_clip_kernel    the apply branch WITH tf.clip_by_global_norm (36 B/elem), optimization.py:80-88,
+//                        128-177: see the block comment above its definition.
 // Arithmetic uses round-to-nearest intrinsics (__fmul_rn, __fadd_rn, __fdiv_rn, __fsqrt_rn) so nvcc
 // cannot contract mul+add into FMA: the reference graph is un-fused, one rounding per TF op, and we
 // reproduce it bit for bit (the kernels are HBM-bound, the extra flops are free).
@@ -85,21 +70,12 @@ struct KernelParams {
   float* accum;
   float* m;
   float* v;
-  double* partials;   // one per CTA (apply with clip)
   float* stats;       // gaccum_stats
-  uint32_t flags;     // kFlag* bits (all of them produce correct results)
   unsigned long long* barrier;  // apply_clip_kernel: monotonic arrival counter of the consumers' grid barrier
   struct LaunchCounters* counters;  // apply_clip_kernel: two sets of per-launch counters (tickets, pool length, norm accumulator)
-  int32_t tmem_tiles;   // apply_clip_kernel: tiles of a' each consumer group parks in Tensor Memory (0..kTmemTiles)
-#ifdef GACCUM_EXPERIMENTS
-  unsigned long long* debug;  // 16 words per CTA: 4 timestamps (ns) + wait-cycle counters (tools/cta_timeline.py)
-#endif
   Scalars sc;
   PtrTable<CAP> tab;
 };
-
-constexpr uint32_t kFlagAssign = 1u;        // accumulate_kernel stores G instead of adding it
-constexpr uint32_t kFlagDynamicPass1 = 2u;  // apply_clip_kernel: pass 1 hands the non-parked tiles out by atomic tickets instead of by position
 
 // ---------------------------------------------------------------------------------------------
 // memory helpers: G is read exactly once -> streaming (evict-first) loads; zeroing the
@@ -198,10 +174,6 @@ __device__ __forceinline__ void accumulate_tile(const TileDesc d, const KernelPa
   if (g == nullptr) return;   // optimization.py:132 -- tensors without a gradient are skipped
   float* __restrict__ a = prm.accum + (size_t)d.soff32 * kSlabAlign;
   const uint32_t len = d.len, tid = threadIdx.x;
-  if (prm.flags & kFlagAssign) {              // gather: a = G (G may live in pinned host memory)
-    for (uint32_t i = tid; i < len; i += kThreads) a[i] = ld_stream(g + i);
-    return;
-  }
   if (aligned16(g)) {
     const uint32_t nvec = len >> 2;
     const float4* g4 = reinterpret_cast<const float4*>(g);
@@ -231,20 +203,10 @@ __device__ __forceinline__ void accumulate_tile(const TileDesc d, const KernelPa
 template <int CAP>
 __global__ void __launch_bounds__(kThreads)
 accumulate_kernel(const __grid_constant__ KernelParams<CAP> prm) {
-  int t = blockIdx.x;
-  if (blockIdx.x == 0 && threadIdx.x == 0 && !(prm.flags & kFlagAssign)) {   // the gather pass is not a step
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
     prm.stats[0] = 0.f; prm.stats[1] = prm.sc.lr; prm.stats[2] = 0.f; prm.stats[3] = 1.f;
   }
-  if (t >= prm.num_tiles) return;
-  TileDesc d = prm.tiles[t];
-  while (true) {
-    const int tn = t + gridDim.x;
-    TileDesc dn;
-    if (tn < prm.num_tiles) dn = prm.tiles[tn];   // prefetch the next descriptor
-    accumulate_tile(d, prm);
-    if (tn >= prm.num_tiles) break;
-    t = tn; d = dn;
-  }
+  if ((int)blockIdx.x < prm.num_tiles) accumulate_tile(prm.tiles[blockIdx.x], prm);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -317,39 +279,10 @@ __device__ __forceinline__ void update_tile(const TileDesc d, const KernelParams
 template <int VARIANT, bool HAS_G, int CAP>
 __global__ void __launch_bounds__(kThreads)
 apply_kernel(const __grid_constant__ KernelParams<CAP> prm) {
-  const int nt = prm.num_tiles;
-  int t = blockIdx.x;
-  if (t < nt) {
-    TileDesc d = prm.tiles[t];
-    while (true) {
-      const int tn = t + gridDim.x;
-      TileDesc dn;
-      if (tn < nt) dn = prm.tiles[tn];
-      update_tile<VARIANT, HAS_G>(d, prm);
-      if (tn >= nt) break;
-      t = tn; d = dn;
-    }
-  }
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     prm.stats[0] = 1.f; prm.stats[1] = prm.sc.lr; prm.stats[2] = 0.f; prm.stats[3] = 1.f;
   }
-}
-
-// Deterministic CTA reduction of one double per thread -> total in thread 0.  Threads add each
-// tile's 8-element fp32 partial into an fp64 running sum, so the norm of a 335 M-element model is
-// good to ~1e-7 relative even for adversarial (constant) data.
-__device__ __forceinline__ double block_reduce_to_double(double x, double* smem /* blockDim.x/32 */) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  if (lane == 0) smem[warp] = x;
-  __syncthreads();
-  double tot = 0.0;
-  if (threadIdx.x == 0) {
-    const int nw = ((int)blockDim.x + 31) >> 5;
-    for (int w = 0; w < nw; ++w) tot += smem[w];
-  }
-  return tot;
+  if ((int)blockIdx.x < prm.num_tiles) update_tile<VARIANT, HAS_G>(prm.tiles[blockIdx.x], prm);
 }
 
 // =============================================================================================
@@ -395,17 +328,13 @@ constexpr int kTmemCols = 512;                    // one CTA per SM: take all co
 constexpr int kTmemColsPerWarp = 80;              // 6 warps share a lane quadrant: 6 x 80 = 480 <= 512
 constexpr int kTmemTiles = kTmemColsPerWarp / 8;  // 10 tiles per group
 constexpr uint32_t kNoTmem = 0xffffffffu;
-#ifndef GACCUM_P1_SLOTS
-#define GACCUM_P1_SLOTS 2
-#endif
-constexpr int kP1Slots = GACCUM_P1_SLOTS;         // pass-1 ring slots per group, 16 KB each
+constexpr int kP1Slots = 2;                       // pass-1 ring slots per group, 16 KB each
 constexpr int kP1SlotVecs = 2 * (kTile / 4);      // float4 per pass-1 slot: G | a
 constexpr int kP2SlotVecs = 4 * (kTile / 4);      // float4 per pass-2 slot: p | m | v | a'
 constexpr int kRingVecs = kP1Slots * kP1SlotVecs; // per group
 constexpr int kP2Slots = kRingVecs / kP2SlotVecs; // 2 x 16 KB = 32 KB -> 1 x 32 KB (deeper rings measured slower: r02_tune_sweep.md)
 constexpr int kRingBytes = kGroups * kRingVecs * 16;   // dynamic shared memory of the kernel (96 KB)
-static_assert(kP2Slots >= 1 && kP1Slots <= 8, "ring must hold at least one [p|m|v|a'] slot");
-constexpr int kMaxSlots = 8;
+static_assert(kP2Slots >= 1, "ring must hold at least one [p|m|v|a'] slot");
 constexpr int kTicketBatch = 4;                   // pass-1 tickets a producer draws at once while plenty of tiles are left
 // what the producer tells the consumers about the tile it put into a slot
 struct __align__(16) SlotMeta {
@@ -683,7 +612,7 @@ __device__ __forceinline__ void update_tile2(const TileDesc& d, const KernelPara
   }
 }
 
-// Dynamic shared memory of apply_clip_kernel: 3 groups x kRingVecs float4 (192 KB).
+// Dynamic shared memory of apply_clip_kernel: 3 groups x kRingVecs float4 (96 KB).
 template <int VARIANT, bool HAS_G, int CAP>
 __global__ void __launch_bounds__(kClipThreads, 1)
 apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
@@ -692,10 +621,10 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
   __shared__ unsigned int s_nonfinite;
   __shared__ float s_bcast[2];
   __shared__ uint32_t s_tmem_base, s_set;
-  __shared__ __align__(8) uint64_t s_full1[kGroups][kMaxSlots], s_empty1[kGroups][kMaxSlots];
-  __shared__ __align__(8) uint64_t s_full2[kGroups][kMaxSlots], s_empty2[kGroups][kMaxSlots];
+  __shared__ __align__(8) uint64_t s_full1[kGroups][kP1Slots], s_empty1[kGroups][kP1Slots];
+  __shared__ __align__(8) uint64_t s_full2[kGroups][kP2Slots], s_empty2[kGroups][kP2Slots];
   __shared__ __align__(8) uint64_t s_go[kGroups];
-  __shared__ SlotMeta s_meta1[kGroups][kMaxSlots], s_meta2[kGroups][kMaxSlots];
+  __shared__ SlotMeta s_meta1[kGroups][kP1Slots], s_meta2[kGroups][kP2Slots];
 
   const int warp = (int)threadIdx.x >> 5;
   const bool is_producer = warp >= kConsumerThreads / 32;
@@ -703,23 +632,10 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
   const int nt = prm.num_tiles, G = (int)gridDim.x * kGroups;
   const int b = (int)blockIdx.x * kGroups + grp;                   // virtual block id
   const int C = b < nt ? (nt - 1 - b) / G + 1 : 0;                 // tiles b, b + G, ... of this group's static share
-  const int n_tm = min(prm.tmem_tiles, C);                         // own tiles: a' parked in Tensor Memory
-  const int pool_lo = min(nt, prm.tmem_tiles * G);                 // tiles [pool_lo, nt): a' goes back to global memory
+  const int n_tm = min(kTmemTiles, C);                             // own tiles: a' parked in Tensor Memory
+  const int pool_lo = min(nt, kTmemTiles * G);                     // tiles [pool_lo, nt): a' goes back to global memory
   float4* const ring = reinterpret_cast<float4*>(smem_dyn) + (size_t)grp * kRingVecs;
   const uint64_t pol_last = policy_evict_last();
-
-#ifdef GACCUM_EXPERIMENTS
-  auto stamp = [&](int which) {
-    if (prm.debug && threadIdx.x == 0) {
-      unsigned long long t;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-      prm.debug[blockIdx.x * 16 + which] = t;
-    }
-  };
-#else
-  auto stamp = [](int) {};
-#endif
-  stamp(0);
 
   // ---- set-up: which counter set this launch uses, mbarriers, accumulator, Tensor Memory ---------------------
   if (threadIdx.x == 0) {
@@ -737,11 +653,11 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   }
   for (int i = threadIdx.x; i < (kConsumerThreads / 32) * kAccBins; i += kClipThreads) (&s_bins[0][0])[i] = 0ull;
-  if (prm.tmem_tiles > 0 && warp == 1) tmem_alloc(&s_tmem_base);
+  if (warp == 1) tmem_alloc(&s_tmem_base);
   asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
   __syncthreads();
   asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-  const uint32_t tmem_base = prm.tmem_tiles > 0 ? s_tmem_base : 0u;
+  const uint32_t tmem_base = s_tmem_base;
   LaunchCounters* const ctr = prm.counters + s_set;
   if (blockIdx.x == 0 && threadIdx.x >= 64 && threadIdx.x < 64 + (int)(sizeof(LaunchCounters) / 8)) {
     // the other set was used by the previous launch on this plan, which is complete: clear it for the next one
@@ -752,15 +668,11 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     // =========================== producer warp of group `grp` ===========================
     const int lane = (int)threadIdx.x & 31;
     const uint64_t pol_first = policy_evict_first();
-#ifdef GACCUM_EXPERIMENTS
-    long long dbg_empty = 0;
-    const long long dbg_p0 = clock64();
-#endif
-    // ---- pass 1.  First the group's OWN tiles b + j*G, j < tmem_tiles: their a' is parked in this SM's Tensor Memory, so
-    //      they are bound to it in both passes.  Then the rest of the model, tiles [pool_lo, nt): either this group's static
-    //      share (b + j*G) or, with kFlagDynamicPass1, whatever the global ticket counter hands out -- kTicketBatch tickets at
-    //      a time while plenty are left (one atomic per lane, the descriptor loads of a batch overlap), single tickets
-    //      near the end so that no SM is left holding a batch ----
+    // ---- pass 1.  First the group's OWN tiles b + j*G, j < n_tm: their a' is parked in this SM's Tensor Memory, so
+    //      they are bound to it in both passes.  Then the rest of the model, tiles [pool_lo, nt), in whatever order the
+    //      global ticket counter hands them out -- kTicketBatch tickets at a time while plenty are left (one atomic per
+    //      lane, the descriptor loads of a batch overlap), single tickets near the end so that no SM is left holding a
+    //      batch ----
     {
       RingPos rp;
       auto issue = [&](const TileDesc& dl, const uint32_t tile) {          // lane 0 only
@@ -768,13 +680,7 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
         if constexpr (HAS_G) g = grad_ptr(prm.tab, dl);
         const uint32_t nvec = bulk_vecs(dl, g);
         uint64_t* full = &s_full1[grp][rp.slot];
-#ifdef GACCUM_EXPERIMENTS
-        const long long t_e0 = clock64();
-#endif
         mbar_wait(&s_empty1[grp][rp.slot], rp.use & 1u);             // the consumers have released the slot
-#ifdef GACCUM_EXPERIMENTS
-        dbg_empty += clock64() - t_e0;
-#endif
         SlotMeta* meta = &s_meta1[grp][rp.slot];
         meta->d = dl;
         meta->tile = tile;
@@ -795,19 +701,17 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
         dl.soff32 = __shfl_sync(0xffffffffu, d.soff32, l);
         return dl;
       };
-      const bool dynamic = (prm.flags & kFlagDynamicPass1) != 0;
-      const int n_static = dynamic ? n_tm : C;                                // tiles b + j*G, j < n_static, are this group's by position
-      for (int j0 = 0; j0 < n_static; j0 += 32) {                              // descriptors 32 at a time, one per lane
+      {
+        static_assert(kTmemTiles <= 32, "one descriptor per lane");
         TileDesc d{};
-        if (j0 + lane < n_static) d = prm.tiles[b + (j0 + lane) * G];
-        const int nb = min(32, n_static - j0);
-        for (int l = 0; l < nb; ++l) {
+        if (lane < n_tm) d = prm.tiles[b + lane * G];
+        for (int l = 0; l < n_tm; ++l) {
           const TileDesc dl = shuffled(d, l);
-          if (lane == 0) issue(dl, (uint32_t)(b + (j0 + l) * G));
+          if (lane == 0) issue(dl, (uint32_t)(b + l * G));
           rp.advance(kP1Slots);
         }
       }
-      bool done = !dynamic;
+      bool done = false;
       long long last = pool_lo;
       while (!done) {
         const long long left = (long long)nt - last;
@@ -840,12 +744,6 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
       }
       __syncwarp();
     }
-#ifdef GACCUM_EXPERIMENTS
-    if (prm.debug && lane == 0) {
-      prm.debug[blockIdx.x * 16 + 7 + grp] = (unsigned long long)dbg_empty;               // cycles the producer waited for a free slot
-      prm.debug[blockIdx.x * 16 + 13 + grp] = (unsigned long long)(clock64() - dbg_p0);   // cycles until pass 1 was issued and drained
-    }
-#endif
     // ---- pass 2.  First the group's own Tensor-Memory tiles (their a' cannot move; their p, m, v do not depend on
     //      the clip scale, so these copies start BEFORE the grid barrier and HBM stays busy while the CTAs wait for
     //      each other).  Then tickets over the pool of L2-resident tiles, youngest first.  Pool tiles carry their a'
@@ -906,10 +804,6 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     __syncwarp();
   } else {
     // =========================== consumer group ===========================
-#ifdef GACCUM_EXPERIMENTS
-    long long dbg_wait = 0;
-    const long long dbg_t0 = clock64();
-#endif
     const bool leader = (threadIdx.x & (kThreads - 1)) == 0;
     // every slot starts out empty: the consumers say so (phase 0 of each `empty` barrier), so that the producer's very
     // first wait is an ordinary wait on a phase that completes -- use u of a slot waits for phase u
@@ -923,16 +817,10 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
       RingPos rp;
       int n_seen = 0;
       while (true) {
-#ifdef GACCUM_EXPERIMENTS
-        const long long t_w0 = clock64();
-#endif
         mbar_wait(&s_full1[grp][rp.slot], rp.use & 1u);
-#ifdef GACCUM_EXPERIMENTS
-        dbg_wait += clock64() - t_w0;
-#endif
         const SlotMeta meta = s_meta1[grp][rp.slot];
         if (meta.d.len == 0) break;
-        // Tensor Memory takes the group's own tiles j < tmem_tiles (the first ones it is handed) when they are FULL,
+        // Tensor Memory takes the group's own tiles j < n_tm (the first ones it is handed) when they are FULL,
         // vector-path tiles (tcgen05.st/ld are warp-collective)
         const bool own = n_seen < n_tm;
         const bool park = own && tmem_ok<HAS_G>(meta.d, prm);
@@ -947,12 +835,6 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
         rp.advance(kP1Slots);
       }
     }
-#ifdef GACCUM_EXPERIMENTS
-    if (prm.debug && leader) {
-      prm.debug[blockIdx.x * 16 + 4 + grp] = (unsigned long long)dbg_wait;                 // cycles waiting for G | a
-      prm.debug[blockIdx.x * 16 + 10 + grp] = (unsigned long long)(clock64() - dbg_t0);   // cycles of the group's pass 1
-    }
-#endif
     named_bar_sync(1, kConsumerThreads);                     // every consumer thread of this CTA is through pass 1
     // flush this CTA's accumulators into the launch's global one (integer adds: order does not matter)
     if (my_nonfinite) atomicOr(&s_nonfinite, my_nonfinite);
@@ -963,7 +845,6 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     }
     named_bar_sync(1, kConsumerThreads);
     if (threadIdx.x == 0 && s_nonfinite) atomicOr(&ctr->nonfinite, s_nonfinite);
-    stamp(1);
     // ---- grid barrier of the consumers: one atomic per CTA on a monotonic counter (every launch of this plan
     //      uses the same grid, so the counter advances by gridDim.x per launch); cooperative launch guarantees
     //      that all CTAs are co-resident ----
@@ -975,7 +856,6 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     }
     named_bar_sync(1, kConsumerThreads);
     if (leader) mbar_arrive(&s_go[grp]);                     // this group's producer may now fetch pool tiles
-    stamp(2);
     // ---- every CTA evaluates the same exact sum the same way: bit-identical gn and clip scale everywhere ----
     if (threadIdx.x < kAccBins) s_bins[0][threadIdx.x] = __ldcg(&ctr->bins[threadIdx.x]);
     named_bar_sync(1, kConsumerThreads);
@@ -1004,8 +884,7 @@ apply_clip_kernel(const __grid_constant__ KernelParams<CAP> prm) {
     }
   }
   __syncthreads();
-  stamp(3);
-  if (prm.tmem_tiles > 0 && warp == 1) tmem_dealloc(tmem_base);
+  if (warp == 1) tmem_dealloc(tmem_base);
 }
 
 }  // namespace gaccum

@@ -15,7 +15,6 @@ not reproduced.)
 """
 from __future__ import annotations
 
-import os
 from typing import Optional, Sequence
 
 import torch
@@ -121,11 +120,10 @@ class FusedDataParallelTrainOp:
             self.comm.param_peers[w] = int(hp_.buffer_ptrs[w])
             self.comm.stage_peers[w] = int(hs_.buffer_ptrs[w])
             self.comm.ctrl_peers[w] = int(hc_.buffer_ptrs[w])
-        if os.environ.get("GACCUM_DP_LOCAL_VA", "1") == "1":
-            # own buffers through their ordinary local mapping, not the peer-aperture alias
-            self.comm.param_peers[self.rank] = self.param_slab.data_ptr()
-            self.comm.stage_peers[self.rank] = self.stage.data_ptr()
-            self.comm.ctrl_peers[self.rank] = self.ctrl.data_ptr()
+        # own buffers through their ordinary local mapping, not the peer-aperture alias
+        self.comm.param_peers[self.rank] = self.param_slab.data_ptr()
+        self.comm.stage_peers[self.rank] = self.stage.data_ptr()
+        self.comm.ctrl_peers[self.rank] = self.ctrl.data_ptr()
         self.tile_lo, self.tile_hi, self.owned_elements = self.plan.dp_shard_range(self.world, self.rank)
         self.epoch = 0
         self.exchanges = 0

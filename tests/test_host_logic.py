@@ -30,6 +30,15 @@ def test_library_has_no_torch_or_oracle_dependency():
     assert "torch" not in out and "oracle" not in out and "python" not in out
 
 
+def test_library_reads_no_gaccum_environment_variables():
+    """Every kernel configuration is fixed at build time: the environment a process inherits cannot select an
+    untested one.  A getenv("GACCUM_...") would leave its name as a NUL-terminated string in the binary."""
+    with open(g.lib_path(), "rb") as f:
+        blob = f.read()
+    names = re.findall(rb"(?<=\x00)GACCUM_[A-Z0-9_]+(?=\x00)", blob)
+    assert not names, f"libgaccum.so names environment variables: {sorted(set(names))}"
+
+
 @pytest.mark.parametrize("sched", [(2e-5, 207900, 20790), (2e-5, 207900, 0), (1e-2, 12, 3), (5e-5, 1000, 100)])
 def test_learning_rate_matches_both_oracles_bitwise(sched):
     init_lr, T, W = sched
